@@ -7,6 +7,7 @@
         bench.py --gpus N --steps K --warmup W                          # one rank per GPU
     ... --config cfg3 | cfg5        # 784 -> 10 logistic on 50M rows / 2-layer MLP 64 -> 32 -> 10 on 10M rows
     ... --scaling weak              # r01 mode: every GPU scores its own 10M rows (default: strong - ONE batch split)
+    ... --dump-outputs DIR          # after the timed steps: DIR/labels.npy, the last timed step's labels (see dump_labels)
 
 A "step" is one pass of the hot path over one batch.  At N > 1 the batch is split across the GPUs (north_star: "the
 batch is split across GPUs", SURVEY.md 8e partition [r*N/G, (r+1)*N/G)), every rank scores its shard in EXACT mode
@@ -36,6 +37,7 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True  # the bench writes nothing into the tree it runs from (it may be read-only)
 
 UNIT = "rows/s"
 CONFIGS = {
@@ -60,6 +62,8 @@ CONFIGS = {
     },
 }
 CHUNK = 1_000_000  # digits rows are generated in global 1M-row chunks: chunk k = default_rng(k)
+DUMP_ALL_ROWS = 12_000_000  # --dump-outputs writes every label up to this many rows (48 MB of float32) ...
+DUMP_SAMPLE_ROWS = 4_000_000  # ... and a seeded sample of this many rows (+ their indices, 48 MB in all) above it
 
 
 # ---------------------------------------------------------------------------------------------------------------
@@ -133,6 +137,23 @@ def float64_labels(cfg, arrs, X64: np.ndarray) -> np.ndarray:
         h = np.maximum(X64 @ arrs["w1"].astype(np.float64).T + arrs["b1"].astype(np.float64), 0.0)
         return (h @ arrs["w2"].astype(np.float64).T + arrs["b2"].astype(np.float64)).argmax(1)
     return (X64 @ arrs["coef"].astype(np.float64).T + arrs["intercept"].astype(np.float64)).argmax(1)
+
+
+def dump_labels(out_dir: str, labels: np.ndarray) -> None:
+    """--dump-outputs: DIR/labels.npy, the class index of every row of the global batch as float32.
+
+    Above DUMP_ALL_ROWS rows it holds a fixed sample instead (DUMP_SAMPLE_ROWS rows drawn by default_rng(0), in row
+    order) and DIR/rows.npy the global row index of each entry (float64).  The inputs are seeded, so two builds run with
+    the same arguments can be compared label for label."""
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    if labels.shape[0] > DUMP_ALL_ROWS:
+        rows = np.sort(np.random.default_rng(0).choice(labels.shape[0], DUMP_SAMPLE_ROWS, replace=False))
+        labels = labels[rows]
+        np.save(out / "rows.npy", rows.astype(np.float64))
+    else:
+        (out / "rows.npy").unlink(missing_ok=True)
+    np.save(out / "labels.npy", labels.astype(np.float32))
 
 
 def measured_peak_hbm():
@@ -557,6 +578,8 @@ def run_gpu_arm(args, cfg):
     # ---- timed region: exactly K steps, CUDA events on the launching stream ----
     ms_per_step = timed_steps(step, args.steps)
     value = G / (ms_per_step * 1e-3)
+    # the labels the last timed step left, copied out before the untimed steps below write the vector again
+    dumped = labels_all.cpu().numpy() if args.dump_outputs and rank == 0 else None
 
     # ---- roofline of the dominant kernel: CUDA events around the scoring kernel inside the library, live ----
     k_ms, r_ms, flagged, launches_per_step, path = [], [], 0, 2, 0
@@ -680,6 +703,8 @@ def run_gpu_arm(args, cfg):
         cpu_baseline = {**extra, "value": rps, "unit": UNIT, "cores": cores, "kind": "port",
                         "sample": cpu_sample_note(cfg, sample, cores) + ", best of 3"}
 
+    if dumped is not None:
+        dump_labels(args.dump_outputs, dumped)
     if rank == 0:
         line = {
             "metric": cfg["metric"], "value": value, "unit": UNIT, "n_gpus": world, "steps": args.steps,
@@ -847,7 +872,13 @@ def main():
     ap.add_argument("--no-multicast", action="store_true", help="per-peer stores instead of the NVLS multicast alias")
     ap.add_argument("--no-graph", action="store_true", help="N > 1: launch every step eagerly instead of replaying a CUDA graph")
     ap.add_argument("--traffic", type=float, default=None, help="dram bytes/launch from a committed ncu capture")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the labels of the last timed step to DIR/labels.npy (float32; a seeded sample of large batches)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
     args.scaling_resolved = "strong" if args.scaling in ("auto", "strong") else "weak"
     cfg = CONFIGS[args.config]
     if args.impl == "reference":
