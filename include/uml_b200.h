@@ -210,6 +210,15 @@ UML_API int uml_mlp_predict_host_begin(uml_engine* e, const uml_mlp* m, const vo
  * path 5); other batches take the CUDA-core kernel (path 3) and a thin scatter kernel. */
 UML_API int uml_mlp_predict_peers(uml_engine* e, const uml_mlp* m, const uml_batch* b, void* const* peer_labels, int n_peers,
                           int64_t row_offset, int label_bytes, int mode, uml_stats* stats);
+/* class probabilities of the MLP: what PytorchModel.forward returns (quickstart.py:14-24), softmax of the logits, fp32
+ * (m = max z, e_c = exp(z_c - m), p_c = e_c / sum e).  The kernel is chosen as for uml_mlp_predict: tensor cores for
+ * batches of tf32 values (stats path 5), CUDA cores for other batches (path 3), an fp64 kernel for shapes neither
+ * takes (path 2).  Rows the fast kernels cannot score (features that are not tf32 values on path 5, NaN/Inf) are
+ * recomputed in fp64 (stats n_flagged).  A row with NaN/Inf returns UML_ERR_NONFINITE, wrapped device rows included.
+ * proba_out: n_rows x n_out row-major fp32, host or (proba_on_device != 0) device memory, 16-byte aligned on the device
+ * (UML_ERR_UNSUPPORTED otherwise).  stats may be NULL; the call is synchronous either way. */
+UML_API int uml_mlp_predict_proba(uml_engine* e, const uml_mlp* m, const uml_batch* b, float* proba_out,
+                                  int proba_on_device, uml_stats* stats);
 
 #ifdef __cplusplus
 }

@@ -48,4 +48,14 @@ X784 = (rng.integers(0, 256, size=(6_001, 784)) / 255.0)
 m784 = eng.load_linear(rng.standard_normal((10, 784)) * 0.05, rng.standard_normal(10))
 eng.predict(m784, eng.stage(X784), exact=True)
 eng.predict_host(m784, X784, exact=True, chunk_rows=2048)
+# MLP class probabilities: softmax epilogues of the tensor-core kernel (tf32 rows) and the CUDA-core kernel (float rows),
+# the fp64 kernel over the flagged rows (rows that are not tf32 values, forced onto the tensor cores) and over all rows
+eng.predict_mlp_proba(mlp, b)
+eng.predict_mlp_proba(mlp, bf)
+_os.environ["UML_B200_MLP_TC"] = "1"
+eng.predict_mlp_proba(mlp, bf)
+del _os.environ["UML_B200_MLP_TC"]
+m48 = eng.load_mlp(rng.standard_normal((48, 64)).astype(np.float32), np.zeros(48, np.float32),
+                   rng.standard_normal((10, 48)).astype(np.float32), np.zeros(10, np.float32))
+eng.predict_mlp_proba(m48, b)
 print("sanitizer driver ok")

@@ -108,6 +108,7 @@ SIGNATURES = {
         [_P, _P, _P, C.c_int64, C.c_int, C.c_int64, C.c_int64, C.c_int, _P, C.c_int, C.c_int64],
     ),
     "uml_mlp_predict_peers": (C.c_int, [_P, _P, _P, _PP, C.c_int, C.c_int64, C.c_int, C.c_int, C.POINTER(Stats)]),
+    "uml_mlp_predict_proba": (C.c_int, [_P, _P, _P, _P, C.c_int, C.POINTER(Stats)]),
 }
 
 _lib = None

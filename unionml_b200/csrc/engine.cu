@@ -1976,4 +1976,85 @@ int uml_mlp_predict_peers(uml_engine* e, const uml_mlp* m, const uml_batch* b, v
   return mlp_predict_common(e, m, b, nullptr, 1, peer_labels, n_peers, row_offset, label_bytes, mode, stats);
 }
 
+// class probabilities of the MLP (PytorchModel.forward): the kernel choice of mlp_predict_common, each tile kernel with
+// its softmax epilogue, and the fp64 kernel behind it for the rows it flags (features that are not tf32 values on the
+// tensor-core path, NaN/Inf anywhere).  Always synchronous: a non-finite row is an error the caller must see.
+int uml_mlp_predict_proba(uml_engine* e, const uml_mlp* m, const uml_batch* b, float* proba_out, int proba_on_device,
+                          uml_stats* stats) {
+  if (!e || !m || !b || (!proba_out && b->n_rows > 0)) return UML_ERR_INVALID;
+  if (b->n_features != m->dm.n_in)
+    UML_FAIL(e, UML_ERR_SHAPE, "X has %d features, but the module is expecting %d features as input.", b->n_features,
+             m->dm.n_in);
+  if (proba_on_device && (reinterpret_cast<uintptr_t>(proba_out) & 15u))
+    UML_FAIL(e, UML_ERR_UNSUPPORTED, "uml_mlp_predict_proba: device proba_out %p is not 16-byte aligned", (void*)proba_out);
+  UML_CUDA(e, cudaSetDevice(e->device));
+  (void)cudaGetLastError();
+  if (stats) memset(stats, 0, sizeof(*stats));
+  if (b->n_rows == 0) return UML_OK;
+  const bool timed = stats != nullptr;
+  int rc;
+  if ((rc = ensure_flags(e, b->n_rows)) != UML_OK) return rc;
+
+  std::string why;  // same choice as mlp_predict_common (UML_B200_MLP_TC=0 / 1 forces it)
+  bool use_tc = b->has_map && uml::mlp_tc_supported(m->dm, &why);
+  if (use_tc) {
+    const char* env = getenv("UML_B200_MLP_TC");
+    if (env && env[0] == '0') use_tc = false;
+    else if (!(env && env[0] == '1')) use_tc = batch_tf32_exact(e, b) == 1;
+  }
+  const bool use_ffma = !use_tc && b->has_map && uml::mlp_tma_supported(m->dm, &why);
+
+  NvtxRange r_all("uml:mlp_predict_proba");
+  const size_t bytes = (size_t)b->n_rows * m->dm.n_classes * 4;
+  struct Scratch {  // device landing buffer of a host-output call
+    float* p = nullptr;
+    ~Scratch() { cudaFree(p); }
+  } scratch;
+  float* d_out = proba_out;
+  if (!proba_on_device) {
+    UML_CUDA(e, cudaMalloc((void**)&scratch.p, bytes));
+    d_out = scratch.p;
+  }
+  FlagList fl{e->d_flag_count, e->d_flag_rows, (int)std::min<int64_t>(e->flag_cap, INT32_MAX), e->d_counters};
+  if (timed) UML_CUDA(e, cudaEventRecord(e->ev[0], e->stream));
+  UML_CUDA(e, cudaMemsetAsync(e->d_counters, 0, 4 * sizeof(unsigned long long), e->stream));
+  UML_CUDA(e, cudaMemsetAsync(e->d_flag_count, 0, sizeof(int), e->stream));
+  int launches = 0, path = 2;
+  if (timed) UML_CUDA(e, cudaEventRecord(e->ev[1], e->stream));
+  if (use_tc || use_ffma) {
+    if (use_tc) {
+      NvtxRange r_score("uml:mlp_proba_tcgen05");
+      uml::MlpTcLaunch out{};
+      out.n_rows = b->n_rows;
+      out.x = b->x;
+      out.ld = b->ld;
+      UML_CUDA(e, uml::launch_mlp_tc_proba(b->map, m->dm, out, d_out, fl, e->info.sm_count, e->stream));
+      path = 5;
+    } else {
+      NvtxRange r_score("uml:mlp_proba_ffma");
+      UML_CUDA(e, uml::launch_mlp_tma(b->map, m->dm, b->x, b->n_rows, nullptr, false, fl, e->info.sm_count, e->stream, d_out));
+      path = 3;
+    }
+    launches += 1;
+    if (timed) UML_CUDA(e, cudaEventRecord(e->ev[2], e->stream));
+    NvtxRange r_rescore("uml:mlp_proba_f64");
+    UML_CUDA(e, uml::launch_mlp_proba_f64(m->dm, b->x, b->ld, b->n_rows, d_out, fl, false, e->info.sm_count, e->stream));
+    launches += 1;
+  } else {
+    NvtxRange r_score("uml:mlp_proba_f64_generic");
+    UML_CUDA(e, uml::launch_mlp_proba_f64(m->dm, b->x, b->ld, b->n_rows, d_out, fl, true, e->info.sm_count, e->stream));
+    launches += 1;
+    if (timed) UML_CUDA(e, cudaEventRecord(e->ev[2], e->stream));
+  }
+  if (timed) UML_CUDA(e, cudaEventRecord(e->ev[3], e->stream));
+  int64_t d2h = 0;
+  if (!proba_on_device) {
+    UML_CUDA(e, cudaMemcpyAsync(proba_out, d_out, bytes, cudaMemcpyDeviceToHost, e->stream));
+    d2h = (int64_t)bytes;
+  }
+  rc = finish_stats(e, stats, b->n_rows, launches, path, timed);
+  if (stats) stats->d2h_bytes = d2h;
+  return rc;
+}
+
 }  // extern "C"

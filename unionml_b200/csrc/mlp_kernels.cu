@@ -10,6 +10,9 @@
 //    rows whose logit margin is inside the propagated fp32 error bound in fp64.
 //  * mlp_rescore_f64_kernel: warp per row, lane per hidden unit, fp64; flagged rows of EXACT mode, or every row for
 //    shapes the tile kernel is not instantiated for.
+//  * PROBA (uml_mlp_predict_proba): the tile kernel's epilogue stores the fp32 softmax of the logits (mlp_proba.cuh)
+//    and flags rows with a non-finite A1; mlp_proba_f64_kernel recomputes those rows, or every row for other shapes,
+//    in fp64.
 //
 // This is CUDA-core fp32 (FFMA): 4 736 flop/row puts the HBM roofline (25 G rows/s) above the FFMA peak, so this kernel
 // is FMA-pipe bound (~0.66 ms per 10M rows at 1.9 GHz).  It serves batches whose features are NOT tf32 values (general
@@ -20,6 +23,7 @@
 #include "uml_common.cuh"
 #include "tma_ring.cuh"
 #include "mlp_rescore.cuh"
+#include "mlp_proba.cuh"
 
 #ifndef UML_MLP_UNROLL_Q
 #define UML_MLP_UNROLL_Q 8  // feature-quad unroll of the layer-1 loop (same-box A/B, EXACT: 1 -> 1.120, 2 -> 1.056, 4 -> 1.023, 8 -> 1.015 ms)
@@ -55,9 +59,10 @@ struct MlpKernelParams {
   int* flag_count;
   int32_t* flag_rows;
   int flag_cap;
+  float* proba;  // PROBA kernels: n_rows x C fp32, 16-byte aligned
 };
 
-template <int H, int C, bool EXACT>
+template <int H, int C, bool EXACT, bool PROBA = false, bool STAGED = false>
 __global__ void __launch_bounds__(kMlpThreads, 1)
 mlp_argmax_tma_kernel(const __grid_constant__ CUtensorMap xmap, const MlpKernelParams p) {
   constexpr int HP = H + 4;
@@ -170,7 +175,7 @@ mlp_argmax_tma_kernel(const __grid_constant__ CUtensorMap xmap, const MlpKernelP
                   h2[j][m * 2 + 1] = fma2(xx, w23, h2[j][m * 2 + 1]);
                 }
               }
-              if (EXACT) {
+              if (EXACT || PROBA) {
                 const float wmax = wrow[H];
 #pragma unroll
                 for (int j = 0; j < R; ++j) a1[j] = fmaf(fabsf(x[j]), wmax, a1[j]);
@@ -220,9 +225,25 @@ mlp_argmax_tma_kernel(const __grid_constant__ CUtensorMap xmap, const MlpKernelP
         for (int j = 0; j < R; ++j)
 #pragma unroll
           for (int c = 0; c < NZ2; ++c) unpack2(z2[j][c], z[j][2 * c], z[j][2 * c + 1]);
+        if constexpr (PROBA) {
+          // ---- softmax, the warp's 32 rows out per j; a non-finite A1 (NaN/Inf feature) goes to the fp64 kernel ----
+          float* strip = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(empty_bar + S) + 15u) & ~static_cast<uintptr_t>(15)) +
+                         warp * 32 * C;
+#pragma unroll
+          for (int j = 0; j < R; ++j) {
+            const long long row0 = tile * kMlpTileRows + half * 64 + 32 * j;
+            float pr[C];
+#pragma unroll
+            for (int c = 0; c < C; ++c) pr[c] = z[j][c];
+            softmax_f32<C>(pr);
+            warp_store_proba<C, STAGED>(pr, p.proba, row0, p.n_rows, lane, strip);
+            flag_list_append(row0 + lane < p.n_rows && !(a1[j] < INFINITY), row0 + lane, p.flag_count, p.flag_rows,
+                             p.flag_cap, lane);
+          }
+        }
         // ---- argmax (first maximum wins), margin guard, label store ----
 #pragma unroll
-        for (int j = 0; j < R; ++j) {
+        for (int j = 0; j < R && !PROBA; ++j) {
           const long long row = tile * kMlpTileRows + half * 64 + lane + 32 * j;
           float best = z[j][0];
           float second = -INFINITY;
@@ -351,12 +372,72 @@ __global__ void __launch_bounds__(256) mlp_rescore_f64_kernel(const MlpRescorePa
   }
 }
 
+// fp64 softmax of flagged rows (all_rows = 0) or of every row: the re-score kernel's block layout and shared-memory
+// image, mlp_rs_proba_rows instead of the arg-max
+struct MlpProbaF64Params {
+  const float* x;
+  long long ld;
+  long long n_rows;
+  const double* pack;
+  int F, H, C;
+  const int* flag_count;
+  const int32_t* flag_rows;
+  int flag_cap;
+  int all_rows;
+  float* proba;
+  unsigned long long* counters;
+};
+
+__global__ void __launch_bounds__(256) mlp_proba_f64_kernel(const MlpProbaF64Params p) {
+  extern __shared__ __align__(16) double rs_smem[];
+  constexpr int R = kMlpRsRows;
+  MlpRsView view = mlp_rs_stage(rs_smem, p.pack, p.F, p.H, p.C);
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  double* xs = rs_smem + mlp_rs_weight_doubles(p.F, p.H, p.C) + warp * mlp_rs_proba_strip_doubles(p.F, p.H, p.C, R);
+  double* hv = xs + (p.F > p.C ? p.F : p.C) * R;
+  __syncthreads();
+  mlp_rs_finish_stage(view);
+
+  pdl_wait_for_predecessor();  // the flag list and the probabilities of the scoring kernel this launch depends on
+  const long long warp_global = (static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
+  const long long warps_total = (static_cast<long long>(gridDim.x) * blockDim.x) >> 5;
+  const long long n = p.all_rows ? p.n_rows : static_cast<long long>(min(*p.flag_count, p.flag_cap));
+  if (!p.all_rows && blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&p.counters[2], static_cast<unsigned long long>(n));
+  for (long long i = warp_global * R; i < n; i += warps_total * R) {
+    const float* xr[R];
+    float* out[R];
+#pragma unroll
+    for (int r = 0; r < R; ++r) {
+      const long long j = i + r < n ? i + r : i;  // unused slots repeat the first row and store nothing
+      const long long row = p.all_rows ? j : static_cast<long long>(p.flag_rows[j]);
+      xr[r] = p.x + row * p.ld;
+      out[r] = i + r < n ? p.proba + row * p.C : nullptr;
+    }
+    bool bad[R];
+    mlp_rs_proba_rows<R>(view, xr, xs, hv, lane, out, bad);
+#pragma unroll
+    for (int r = 0; r < R; ++r)
+      if (lane == 0 && bad[r] && i + r < n) atomicAdd(&p.counters[1], 1ull);
+  }
+  // hand the flag list back empty (see rescore_f64_kernel in linear_kernels.cu)
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    __threadfence();
+    const unsigned long long ticket = atomicAdd(&p.counters[3], 1ull);
+    if (ticket == static_cast<unsigned long long>(gridDim.x) - 1ull) {
+      *const_cast<int*>(p.flag_count) = 0;
+      p.counters[3] = 0ull;
+      __threadfence();
+    }
+  }
+}
+
 // ---------------------------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------------------------
-static size_t mlp_fixed_smem(const MlpDeviceModel& m) {
+static size_t mlp_fixed_smem(const MlpDeviceModel& m, bool proba = false) {
   return 1024 + (static_cast<size_t>(m.f_pad) * (m.n_hidden + 4) + (m.n_hidden + 4) + static_cast<size_t>(m.n_hidden) * m.cp + m.cp) * 4 +
-         2 * 64 * 8;
+         2 * 64 * 8 + (proba ? 16 + static_cast<size_t>(kMlpConsumerWarps) * 32 * m.n_classes * 4 : 0);  // + output strips
 }
 
 bool mlp_tma_supported(const MlpDeviceModel& m, std::string* why) {
@@ -372,10 +453,10 @@ bool mlp_tma_supported(const MlpDeviceModel& m, std::string* why) {
   return true;
 }
 
-template <int H, int C, bool EXACT>
+template <int H, int C, bool EXACT, bool PROBA = false, bool STAGED = false>
 static cudaError_t mlp_launch_one(const CUtensorMap& xmap, const MlpKernelParams& p, int grid, size_t smem,
                                   cudaStream_t stream) {
-  auto kern = mlp_argmax_tma_kernel<H, C, EXACT>;
+  auto kern = mlp_argmax_tma_kernel<H, C, EXACT, PROBA, STAGED>;
   static size_t configured = 0;
   if (smem > configured) {
     cudaError_t err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
@@ -396,8 +477,20 @@ static cudaError_t mlp_dispatch(int H, int C, const CUtensorMap& xmap, const Mlp
   return cudaErrorInvalidValue;
 }
 
+template <bool STAGED>
+static cudaError_t mlp_dispatch_proba(int H, int C, const CUtensorMap& xmap, const MlpKernelParams& p, int grid,
+                                      size_t smem, cudaStream_t stream) {
+#define UML_MLP_CASE(HH, CC) \
+  if (H == HH && C == CC) return mlp_launch_one<HH, CC, false, true, STAGED>(xmap, p, grid, smem, stream);
+  UML_MLP_CASE(32, 10) UML_MLP_CASE(32, 2) UML_MLP_CASE(32, 3) UML_MLP_CASE(16, 10) UML_MLP_CASE(16, 2) UML_MLP_CASE(16, 3)
+#undef UML_MLP_CASE
+  return cudaErrorInvalidValue;
+}
+
+// proba != nullptr: the PROBA kernel (softmax epilogue into proba, non-finite rows to the flag list); labels unused
 cudaError_t launch_mlp_tma(const CUtensorMap& xmap, const MlpDeviceModel& m, const float* x, int64_t n_rows,
-                           int32_t* labels, bool exact, const FlagList& flags, int sm_count, cudaStream_t stream) {
+                           int32_t* labels, bool exact, const FlagList& flags, int sm_count, cudaStream_t stream,
+                           float* proba) {
   (void)x;
   if (n_rows <= 0) return cudaSuccess;
   MlpKernelParams p{};
@@ -410,7 +503,7 @@ cudaError_t launch_mlp_tma(const CUtensorMap& xmap, const MlpDeviceModel& m, con
   p.num_tiles = (n_rows + kMlpTileRows - 1) / kMlpTileRows;
   p.f_pad = m.f_pad;
   p.kc = m.f_pad / kChunkF;
-  const size_t fixed = mlp_fixed_smem(m);
+  const size_t fixed = mlp_fixed_smem(m, proba != nullptr);
   int stages = static_cast<int>((static_cast<size_t>(kMaxSmemBytes) - fixed) / kMlpStageBytes);
   stages = std::min(stages, 64);
   if (const char* env = getenv("UML_B200_STAGES")) stages = std::max(kMlpPairs, std::min(stages, atoi(env)));
@@ -422,9 +515,13 @@ cudaError_t launch_mlp_tma(const CUtensorMap& xmap, const MlpDeviceModel& m, con
   p.flag_count = flags.count;
   p.flag_rows = flags.rows;
   p.flag_cap = flags.capacity;
+  p.proba = proba;
   const size_t smem = fixed + static_cast<size_t>(stages) * kMlpStageBytes;
   const long long slots = (p.num_tiles + kMlpPairs - 1) / kMlpPairs;
   const int grid = static_cast<int>(std::min<long long>(sm_count, std::max<long long>(1, slots)));
+  if (proba)
+    return mlp_proba_staged_store() ? mlp_dispatch_proba<true>(m.n_hidden, m.n_classes, xmap, p, grid, smem, stream)
+                                    : mlp_dispatch_proba<false>(m.n_hidden, m.n_classes, xmap, p, grid, smem, stream);
   return exact ? mlp_dispatch<true>(m.n_hidden, m.n_classes, xmap, p, grid, smem, stream)
                : mlp_dispatch<false>(m.n_hidden, m.n_classes, xmap, p, grid, smem, stream);
 }
@@ -465,6 +562,41 @@ cudaError_t launch_mlp_rescore_f64(const MlpDeviceModel& m, const float* x, int6
   long long blocks = static_cast<long long>(sm_count) * per_sm;  // persistent: every resident warp loops over rows
   if (all_rows) blocks = std::min<long long>(blocks, (n_rows + 8 * kMlpRsRows - 1) / (8 * kMlpRsRows));
   cudaError_t lerr = launch_dependent(mlp_rescore_f64_kernel, static_cast<int>(std::max<long long>(1, blocks)), 256, smem, stream, p);
+  if (lerr != cudaSuccess) return lerr;
+  return cudaGetLastError();
+}
+
+cudaError_t launch_mlp_proba_f64(const MlpDeviceModel& m, const float* x, int64_t ld, int64_t n_rows, float* proba,
+                                 const FlagList& flags, bool all_rows, int sm_count, cudaStream_t stream) {
+  if (n_rows <= 0) return cudaSuccess;
+  MlpProbaF64Params p{};
+  p.x = x;
+  p.ld = ld;
+  p.n_rows = n_rows;
+  p.pack = m.rs_pack;
+  p.F = m.n_in;
+  p.H = m.n_hidden;
+  p.C = m.n_classes;
+  p.flag_count = flags.count;
+  p.flag_rows = flags.rows;
+  p.flag_cap = flags.capacity;
+  p.all_rows = all_rows ? 1 : 0;
+  p.proba = proba;
+  p.counters = flags.counters;
+  const size_t smem = (mlp_rs_weight_doubles(m.n_in, m.n_hidden, m.n_classes) +
+                       8 * mlp_rs_proba_strip_doubles(m.n_in, m.n_hidden, m.n_classes, kMlpRsRows)) * sizeof(double);
+  if (smem > static_cast<size_t>(kMaxSmemBytes)) return cudaErrorInvalidValue;
+  static size_t configured = 0;
+  if (smem > configured) {
+    cudaError_t err = cudaFuncSetAttribute(mlp_proba_f64_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
+    if (err != cudaSuccess) return err;
+    configured = smem;
+  }
+  int per_sm = 0;
+  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mlp_proba_f64_kernel, 256, smem) != cudaSuccess || per_sm < 1) per_sm = 1;
+  long long blocks = static_cast<long long>(sm_count) * per_sm;
+  if (all_rows) blocks = std::min<long long>(blocks, (n_rows + 8 * kMlpRsRows - 1) / (8 * kMlpRsRows));
+  cudaError_t lerr = launch_dependent(mlp_proba_f64_kernel, static_cast<int>(std::max<long long>(1, blocks)), 256, smem, stream, p);
   if (lerr != cudaSuccess) return lerr;
   return cudaGetLastError();
 }

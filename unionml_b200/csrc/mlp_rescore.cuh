@@ -117,15 +117,16 @@ struct MlpRowResult {
   bool ambiguous;  // fp64 logit margin inside the fp64 rounding bound (a true tie; first index wins)
 };
 
-// One warp, R rows per pass.  xr[r] = row r's fp32 features in global memory (callers pass a valid row for unused
-// slots and ignore that result); xs / hv = the warp's strip, F x R and H x R doubles, 16-byte aligned.
+// Layer 1 of R rows on one warp: features -> xs ([f][R] doubles), ReLU'd hidden values -> hv ([n][R]).  xr[r] = row
+// r's fp32 features in global memory (callers pass a valid row for unused slots and ignore that result).  Returns per
+// row: NaN/Inf in the features, a hidden unit's own fp64 rounding bound (herr) and the bound on every logit's absolute
+// sum (amax).
 template <int R>
-__device__ __forceinline__ void mlp_rs_rows(const MlpRsView& v, const float* const (&xr)[R], double* xs, double* hv, int lane,
-                                            MlpRowResult (&out)[R]) {
+__device__ __forceinline__ void mlp_rs_hidden(const MlpRsView& v, const float* const (&xr)[R], double* xs, double* hv, int lane,
+                                              bool (&bad)[R], double (&herr)[R], double (&amax)[R]) {
   static_assert(R == 1 || R == 2 || R == 4, "rows per pass");
   const double u = 1.1102230246251565e-16;  // 2^-53
-  const int F = v.F, H = v.H, C = v.C, HP = v.H + 1;
-  bool bad[R];
+  const int F = v.F, H = v.H;
   double a1[R];  // sum_f |x_f| max_n |w1_nf|: bounds every hidden unit's absolute sum (one chain instead of H)
 #pragma unroll
   for (int r = 0; r < R; ++r) {
@@ -145,7 +146,6 @@ __device__ __forceinline__ void mlp_rs_rows(const MlpRsView& v, const float* con
       a1[r] = fma(fabs(xd), wm, a1[r]);
     }
   }
-  double herr[R];
 #pragma unroll
   for (int r = 0; r < R; ++r) {
     bad[r] = __any_sync(0xffffffffu, bad[r]);
@@ -184,10 +184,21 @@ __device__ __forceinline__ void mlp_rs_rows(const MlpRsView& v, const float* con
       a2[r] = fma(h, wm, a2[r]);
     }
   }
-  double amax[R];
 #pragma unroll
   for (int r = 0; r < R; ++r) amax[r] = warp_sum(a2[r]) + herr[r] * v.w2sum + v.b2max;
   __syncwarp();
+}
+
+// One warp, R rows per pass: arg-max and runner-up of the fp64 logits.  xs / hv = the warp's strip, F x R and H x R
+// doubles, 16-byte aligned.
+template <int R>
+__device__ __forceinline__ void mlp_rs_rows(const MlpRsView& v, const float* const (&xr)[R], double* xs, double* hv, int lane,
+                                            MlpRowResult (&out)[R]) {
+  const double u = 1.1102230246251565e-16;  // 2^-53
+  const int H = v.H, C = v.C, HP = v.H + 1;
+  bool bad[R];
+  double herr[R], amax[R];
+  mlp_rs_hidden<R>(v, xr, xs, hv, lane, bad, herr, amax);
   // ---- output layer: lane per class, one chain per row over the hidden units ----
   Top2 top[R];
   for (int c0 = 0; c0 < C; c0 += 32) {
@@ -240,6 +251,50 @@ __device__ __forceinline__ void mlp_rs_rows(const MlpRsView& v, const float* con
     const double err = herr[r] * v.w2sum + (static_cast<double>(H) + 16.0) * u * amax[r];
     out[r].ambiguous = !((top[r].best - top[r].second) > 2.0 * err);
   }
+}
+
+// doubles of a warp's strip for mlp_rs_proba_rows: the logits reuse the feature area once layer 1 is done with it
+__host__ __device__ inline size_t mlp_rs_proba_strip_doubles(int F, int H, int C, int R) {
+  return (static_cast<size_t>(F > C ? F : C) + H) * R;
+}
+
+// One warp, R rows per pass: softmax of the fp64 logits, rounded once to fp32 into out[r][0..C) (out[r] == nullptr:
+// unused slot).  xs: max(F, C) x R doubles, hv: H x R, 16-byte aligned.  bad[r]: NaN/Inf in row r's features.
+template <int R>
+__device__ __forceinline__ void mlp_rs_proba_rows(const MlpRsView& v, const float* const (&xr)[R], double* xs, double* hv,
+                                                  int lane, float* const (&out)[R], bool (&bad)[R]) {
+  const int H = v.H, C = v.C, HP = v.H + 1;
+  double herr[R], amax[R];
+  mlp_rs_hidden<R>(v, xr, xs, hv, lane, bad, herr, amax);
+  // ---- output layer: lane per class, logits -> xs ([c][R]) ----
+  for (int c = lane; c < C; c += 32) {
+    double s[R];
+#pragma unroll
+    for (int r = 0; r < R; ++r) s[r] = 0.0;
+    const double* w2c = v.w2s + c * HP;
+#pragma unroll 4
+    for (int nn = 0; nn < H; ++nn) {
+      const double w = w2c[nn];
+#pragma unroll
+      for (int r = 0; r < R; ++r) s[r] = fma(hv[nn * R + r], w, s[r]);
+    }
+#pragma unroll
+    for (int r = 0; r < R; ++r) xs[c * R + r] = s[r] + v.b2s[c];
+  }
+  __syncwarp();
+  // ---- softmax per row: max, sum of exp, one division ----
+#pragma unroll
+  for (int r = 0; r < R; ++r) {
+    double m = -INFINITY;
+    for (int c = lane; c < C; c += 32) m = fmax(m, xs[c * R + r]);
+    m = warp_max(m, 1);
+    double sum = 0.0;
+    for (int c = lane; c < C; c += 32) sum += exp(xs[c * R + r] - m);
+    sum = warp_sum(sum);
+    if (out[r] != nullptr)
+      for (int c = lane; c < C; c += 32) out[r][c] = static_cast<float>(exp(xs[c * R + r] - m) / sum);
+  }
+  __syncwarp();  // the strip may be reused by the caller's next pass
 }
 
 // one row (the re-score warps inside the tensor-core kernel take rows one at a time from their queue)

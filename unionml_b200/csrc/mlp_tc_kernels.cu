@@ -28,6 +28,11 @@
 //   warps 4-11: epilogue    - two sets of four warps taking alternate tiles (the first ncu capture showed one set
 //             80 % busy and everything else waiting on it): tcgen05.ld the row's 2H accumulators, + b1, ReLU, layer 2
 //             from constant-bank operands, argmax (first maximum wins), margin guard, label store (+ peer stores)
+//
+// PROBA kernels (uml_mlp_predict_proba) share the producer, MMA and scan roles; their epilogue turns the same C logits
+// into an fp32 softmax and stores C floats per row (mlp_proba.cuh).  There is no margin guard; rows the MMA cannot
+// score (features that are not tf32 values, or a non-finite A1) go to the flag list and mlp_proba_f64_kernel
+// recomputes them.
 #include <algorithm>
 #include <cstdlib>
 #include <cstring>
@@ -36,12 +41,17 @@
 #include "uml_common.cuh"
 #include "tcgen05.cuh"
 #include "mlp_rescore.cuh"
+#include "mlp_proba.cuh"
 
 #ifndef UML_MLP_QUEUE_DEFAULT
 // 0: the queue variant lost the same-box A/B (profiles/r02_ab.json: 10M rows 0.640 vs 0.577 ms per step) - the scoring
 // kernel is issue-bound (68 % issue slots), so the 58 000 fp64 rows it takes in slow the pipeline by more than the
 // separate re-score kernel costs.  (The linear tile kernel, with 0.02 % flagged rows, wins with its queue.)
 #define UML_MLP_QUEUE_DEFAULT 0
+#endif
+
+#ifndef UML_MLP_PROBA_STAGED_DEFAULT
+#define UML_MLP_PROBA_STAGED_DEFAULT 0
 #endif
 
 namespace uml {
@@ -89,6 +99,7 @@ struct MlpTcParams {
   int n_in;
   const double* rs_pack;  // shared-memory image of the fp64 operands (mlp_rs_build_pack)
   unsigned long long* counters;  // [0] ambiguous, [1] nonfinite, [2] re-scored rows
+  float* proba;  // PROBA kernels: n_rows x C fp32, 16-byte aligned
 };
 
 template <int H, int C>
@@ -100,7 +111,7 @@ __device__ __forceinline__ void tc_store_final_label(const MlpTcParams<H, C>& p,
   }
 }
 
-template <int H, int C, bool EXACT, bool QUEUE>
+template <int H, int C, bool EXACT, bool QUEUE, bool PROBA = false, bool STAGED = false>
 __global__ void __launch_bounds__(kTcThreadsQueue, 1)
 mlp_argmax_tc_kernel(const __grid_constant__ CUtensorMap xmap, const __grid_constant__ MlpTcParams<H, C> p) {
   constexpr int N = 2 * H;  // accumulator columns per tile: [main | small]
@@ -237,7 +248,7 @@ mlp_argmax_tc_kernel(const __grid_constant__ CUtensorMap xmap, const __grid_cons
 #pragma unroll
         for (int q = 0; q < kChunkF / 4; ++q) {
           const float4 v = *reinterpret_cast<const float4*>(xs + rowbase + ((static_cast<uint32_t>(q) * 16u) ^ sw));
-          if (EXACT) {
+          if (EXACT || PROBA) {
             const float* wm = p.w1max + k * kChunkF + q * 4;
             a1 = fmaf(fabsf(v.x), wm[0], a1);
             a1 = fmaf(fabsf(v.y), wm[1], a1);
@@ -300,6 +311,14 @@ mlp_argmax_tc_kernel(const __grid_constant__ CUtensorMap xmap, const __grid_cons
         for (int c = 0; c < NZ; ++c) z[c] = fmaf(hv, p.w2[n][c], z[c]);
       }
       const long long row = tile * kTileRows + row_in_tile;
+      if constexpr (PROBA) {
+        // softmax, the warp's 32 rows out; rows the MMA could not score (A1 = +inf / NaN) are recomputed in fp64
+        softmax_f32<C>(z);
+        float* strip = reinterpret_cast<float*>(rs_area) + (warp - 4) * 32 * C;
+        warp_store_proba<C, STAGED>(z, p.proba, tile * kTileRows + wq * 32, p.n_rows, lane, strip);
+        flag_list_append(row < p.n_rows && !(a1 < INFINITY), row, p.flag_count, p.flag_rows, p.flag_cap, lane);
+        continue;
+      }
       float best = z[0];
       float second = -INFINITY;
       int idx = 0;
@@ -484,10 +503,12 @@ std::vector<float> mlp_tc_build_w1_tiles(const float* w1 /*[H][F]*/, int H, int 
   return tiles;
 }
 
-static size_t mlp_tc_fixed_smem(const MlpDeviceModel& m, bool queue) {
+static size_t mlp_tc_fixed_smem(const MlpDeviceModel& m, bool queue, bool proba = false) {
   const size_t kc = m.f_pad / kChunkF;
   size_t bytes = 1024 + kc * (2 * m.n_hidden) * 128 + static_cast<size_t>(kTcSlots) * kTileRows * 4 +
                  (2 * 64 + 2 * kTcAccStages + kTcSlots) * 8 + 16;
+  if (proba)  // (queue control words, unused) + one 32-row output strip per epilogue warp
+    bytes += (kTcQueueCap + 4) * 4 + 16 + static_cast<size_t>(kTcEpilogueWarps) * 32 * m.n_classes * 4;
   if (queue)  // flagged-row queue + fp64 weights + one strip per epilogue / re-score warp
     bytes += (kTcQueueCap + 4) * 4 + 16 +
              (mlp_rs_weight_doubles(m.n_in, m.n_hidden, m.n_classes) +
@@ -520,9 +541,9 @@ bool mlp_tc_supported(const MlpDeviceModel& m, std::string* why) {
   return mlp_tc_fixed_smem(m, true) + 6 * static_cast<size_t>(kStageBytes) <= static_cast<size_t>(kMaxSmemBytes);
 }
 
-template <int H, int C, bool EXACT, bool QUEUE>
+template <int H, int C, bool EXACT, bool QUEUE, bool PROBA = false, bool STAGED = false>
 static cudaError_t mlp_tc_launch_one(const CUtensorMap& xmap, const MlpDeviceModel& m, const MlpTcLaunch& l,
-                                     const FlagList& flags, int sm_count, cudaStream_t stream) {
+                                     const FlagList& flags, int sm_count, cudaStream_t stream, float* proba = nullptr) {
   using Params = MlpTcParams<H, C>;
   static_assert(sizeof(Params) < 4000, "kernel parameters must stay below the 4 KiB limit");
   Params p;
@@ -569,7 +590,8 @@ static cudaError_t mlp_tc_launch_one(const CUtensorMap& xmap, const MlpDeviceMod
   p.n_in = m.n_in;
   p.rs_pack = m.rs_pack;
   p.counters = flags.counters;
-  const size_t fixed = mlp_tc_fixed_smem(m, QUEUE);
+  p.proba = proba;
+  const size_t fixed = mlp_tc_fixed_smem(m, QUEUE, PROBA);
   int stages = static_cast<int>((static_cast<size_t>(kMaxSmemBytes) - fixed) / kStageBytes);
   stages = std::min(stages, 64);
   if (const char* env = getenv("UML_B200_STAGES")) stages = std::max(4, std::min(stages, atoi(env)));
@@ -580,7 +602,7 @@ static cudaError_t mlp_tc_launch_one(const CUtensorMap& xmap, const MlpDeviceMod
   p.flag_rows = flags.rows;
   p.flag_cap = flags.capacity;
   const size_t smem = fixed + static_cast<size_t>(stages) * kStageBytes;
-  auto kern = mlp_argmax_tc_kernel<H, C, EXACT, QUEUE>;
+  auto kern = mlp_argmax_tc_kernel<H, C, EXACT, QUEUE, PROBA, STAGED>;
   static size_t configured = 0;
   if (smem > configured) {
     cudaError_t err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
@@ -603,6 +625,31 @@ cudaError_t launch_mlp_tc(const CUtensorMap& xmap, const MlpDeviceModel& m, cons
     return queue ? mlp_tc_launch_one<HH, CC, true, true>(xmap, m, l, flags, sm_count, stream)                    \
                  : mlp_tc_launch_one<HH, CC, true, false>(xmap, m, l, flags, sm_count, stream);                  \
   }
+  UML_TC_CASE(32, 10) UML_TC_CASE(32, 2) UML_TC_CASE(32, 3) UML_TC_CASE(16, 10) UML_TC_CASE(16, 2) UML_TC_CASE(16, 3)
+#undef UML_TC_CASE
+  return cudaErrorInvalidValue;
+}
+
+bool mlp_proba_staged_store() {
+  // UML_B200_MLP_PROBA_STORE=staged: probabilities leave through a shared-memory strip as coalesced 16-byte stores;
+  // =direct: every lane stores its own row (DESIGN.md 3.6 has the same-box A/B behind the default)
+  static const int mode = [] {
+    const char* env = getenv("UML_B200_MLP_PROBA_STORE");
+    if (env && env[0] == 's') return 1;
+    if (env && env[0] == 'd') return 0;
+    return UML_MLP_PROBA_STAGED_DEFAULT;
+  }();
+  return mode == 1;
+}
+
+cudaError_t launch_mlp_tc_proba(const CUtensorMap& xmap, const MlpDeviceModel& m, const MlpTcLaunch& l, float* proba,
+                                const FlagList& flags, int sm_count, cudaStream_t stream) {
+  if (l.n_rows <= 0) return cudaSuccess;
+  const bool staged = mlp_proba_staged_store();
+#define UML_TC_CASE(HH, CC)                                                                                        \
+  if (m.n_hidden == HH && m.n_classes == CC)                                                                       \
+    return staged ? mlp_tc_launch_one<HH, CC, false, false, true, true>(xmap, m, l, flags, sm_count, stream, proba) \
+                  : mlp_tc_launch_one<HH, CC, false, false, true, false>(xmap, m, l, flags, sm_count, stream, proba);
   UML_TC_CASE(32, 10) UML_TC_CASE(32, 2) UML_TC_CASE(32, 3) UML_TC_CASE(16, 10) UML_TC_CASE(16, 2) UML_TC_CASE(16, 3)
 #undef UML_TC_CASE
   return cudaErrorInvalidValue;

@@ -150,8 +150,11 @@ struct MlpTcLaunch {
   long long ld;
 };
 bool mlp_tma_supported(const MlpDeviceModel& m, std::string* why);
+// proba != nullptr: the softmax epilogue (n_rows x n_classes fp32 into proba, 16-byte aligned) instead of labels; rows
+// with a non-finite A1 are appended to flags for launch_mlp_proba_f64
 cudaError_t launch_mlp_tma(const CUtensorMap& xmap, const MlpDeviceModel& m, const float* x, int64_t n_rows,
-                           int32_t* labels, bool exact, const FlagList& flags, int sm_count, cudaStream_t stream);
+                           int32_t* labels, bool exact, const FlagList& flags, int sm_count, cudaStream_t stream,
+                           float* proba = nullptr);
 cudaError_t launch_mlp_rescore_f64(const MlpDeviceModel& m, const float* x, int64_t ld, int64_t n_rows,
                                    const MlpTcLaunch& out, const FlagList& flags, bool all_rows, int sm_count,
                                    cudaStream_t stream);
@@ -159,6 +162,14 @@ bool mlp_tc_supported(const MlpDeviceModel& m, std::string* why);
 std::vector<float> mlp_tc_build_w1_tiles(const float* w1, int H, int F, int f_pad);
 cudaError_t launch_mlp_tc(const CUtensorMap& xmap, const MlpDeviceModel& m, const MlpTcLaunch& l, bool exact,
                           const FlagList& flags, int sm_count, cudaStream_t stream, bool* rescore_kernel_needed);
+// class probabilities (uml_mlp_predict_proba): the tensor-core kernel with the softmax epilogue; rows whose features
+// are not tf32 values or whose A1 is not finite are appended to flags.  launch_mlp_proba_f64 recomputes the flagged
+// rows (all_rows = false) or every row (shapes neither tile kernel takes) in fp64 and rounds once to fp32.
+cudaError_t launch_mlp_tc_proba(const CUtensorMap& xmap, const MlpDeviceModel& m, const MlpTcLaunch& l, float* proba,
+                                const FlagList& flags, int sm_count, cudaStream_t stream);
+cudaError_t launch_mlp_proba_f64(const MlpDeviceModel& m, const float* x, int64_t ld, int64_t n_rows, float* proba,
+                                 const FlagList& flags, bool all_rows, int sm_count, cudaStream_t stream);
+bool mlp_proba_staged_store();  // store scheme of the probability epilogues (mlp_proba.cuh: warp_store_proba)
 // int32 labels (device) -> every target vector of a fused exchange (int32 or uint8 wire), for kernels without peer stores
 cudaError_t launch_labels_scatter(const int32_t* labels, int64_t n, void* const* peers, int n_peers, int wire_u8,
                                   int64_t row_offset, int sm_count, cudaStream_t stream);

@@ -276,6 +276,21 @@ class Engine:
             self._check(st)  # under the lock: uml_last_error is per engine, another thread's call may overwrite it
         return out, stats.as_dict() if stats else None
 
+    def predict_mlp_proba(self, model: MlpModel, batch: Batch, out_device_ptr: Optional[int] = None
+                          ) -> Tuple[Optional[np.ndarray], dict]:
+        """``softmax(W2 relu(W1 x + b1) + b2)`` per row, fp32 ``(n_rows, n_out)``: what ``PytorchModel.forward``
+        returns.  Host result unless ``out_device_ptr`` (16-byte aligned device memory) is given."""
+        stats = N.Stats()
+        with self._lock:
+            if out_device_ptr is not None:
+                self._check(N.lib().uml_mlp_predict_proba(self._h, model._h, batch._h, C.c_void_p(out_device_ptr), 1,
+                                                          C.byref(stats)))
+                return None, stats.as_dict()
+            out = np.empty((batch.n_rows, model.n_classes), dtype=np.float32)
+            self._check(N.lib().uml_mlp_predict_proba(self._h, model._h, batch._h, out.ctypes.data_as(C.c_void_p), 0,
+                                                      C.byref(stats)))
+        return out, stats.as_dict()
+
     def predict_mlp_peers(self, model: MlpModel, batch: Batch, peer_ptrs, row_offset: int, exact: bool = True,
                           want_stats: bool = False, label_bytes: int = 4) -> Optional[dict]:
         """Fused compute + all-gather for the MLP predictor (same contract as :meth:`predict_peers`)."""

@@ -327,3 +327,21 @@ def mlp_argmax(module: Any, features: Any) -> List[float]:
     out, stats = engine.predict_host_list(dm, arr, dm.class_table, exact=_exact_default())
     _note_ambiguous(stats)
     return out
+
+
+def mlp_predict_proba(module: Any, features: Any) -> np.ndarray:
+    """``module(process_features(features))`` of the torch quickstart on the GPU: float32 class probabilities,
+    ``(n_rows, n_out)``.  The result is the softmax of the logits ``W2 relu(W1 x + b1) + b2`` whether or not the
+    module's own ``forward`` applies one.  Features are cast to float32 as ``process_features`` does; the whole batch is
+    staged in HBM for the call (as ``linear_predict_proba`` does) and freed afterwards."""
+    engine = get_engine()
+    dm = device_mlp(module, engine)
+    arr = features.to_numpy() if hasattr(features, "to_numpy") else np.asarray(features)
+    _check_min_samples(arr)
+    batch = engine.stage(arr, keep_f64=False)
+    try:
+        proba, stats = engine.predict_mlp_proba(dm, batch)
+    finally:
+        batch.free()
+    _note_ambiguous(stats)
+    return proba
